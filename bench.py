@@ -17,6 +17,15 @@ sharded path instead (one sub-graph per shard, NCCL all-gather + top-k merge).
 Prints ONE JSON line (rank 0).  Inputs (corpus, queries, .graph) are generated once and cached
 in $HS_DATA_CACHE (default /tmp/hs_data_cache); the .graph is built by the engine's own host
 builder (hs_build_slim_graph), not by anything under oracle/.
+
+`--dump-outputs DIR` writes what the last timed step returned (rank 0) as DIR/<name>.npy: the
+labels (as float64, exact) and distances (float32) of the whole batch, and DIR/inputs.json with
+SHA-256 digests of the index and of the query batch.  Corpus and queries are seeded, and the
+.graph is then built deterministically (the multi-threaded host build differs from run to run) and
+cached as its own file: by the GPU builder (about 2 s at 1M x 128), for hnsw_slimq by the host
+builder on one thread (more than 8 minutes at 1M rows).  So two builds of the project run with the
+same arguments search the same inputs and can be compared output for output.  Indices that live
+in HBM only (the sharded and ef-sweep workloads) are digested through hs_save_index.
 """
 from __future__ import annotations
 
@@ -84,18 +93,24 @@ def env_rank():
     return int(os.environ.get("RANK", "0")), int(os.environ.get("LOCAL_RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
 
 
-def prepare_inputs(w: dict, n_query_batches: int, build_rank: bool, reference_builder: bool = False):
+def prepare_inputs(w: dict, n_query_batches: int, build_rank: bool, reference_builder: bool = False,
+                   deterministic: bool = False, device: int = 0):
     """Synthetic corpus + query batches + the .graph over the corpus (cached on disk).  The reference arm
     (reference_builder=True, `--impl reference`, which the driver runs first on a box) builds the hnsw_slim
     graph with the REFERENCE's own builder (addPoint loop + convertFromHNSW through oracle/_ref), so that both
     arms search the graph BASELINE.md specifies; the engine's arm never executes oracle/: it takes the cached
     file, or builds one with its own host builder (profiles/r02_refgraph_probe.txt: same recall and QPS on
-    reference-built, host-built and GPU-built graphs)."""
+    reference-built, host-built and GPU-built graphs).  deterministic=True (--dump-outputs): the .graph is the
+    same file on every machine, cached under its own name: built by the GPU builder (levels drawn from a seed,
+    atomics only for statistics) and saved with hs_save_index, or for hnsw_slimq by the host builder on one
+    thread (its GPU path clusters on all host threads)."""
     from hnsw_slim_b200 import capi
     from hnsw_slim_b200.synth import latent_gaussian
     os.makedirs(CACHE, exist_ok=True)
-    tag = f"n{w['n']}_d{w['dim']}_m{w['metric']}_r{w['rank']}_M{w['M']}_e{w['efc']}_b4_s1"
     slimq = w.get("kind") == "slimq"
+    tag = (f"n{w['n']}_d{w['dim']}_m{w['metric']}_r{w['rank']}_M{w['M']}_e{w['efc']}_b4_s1"
+           + (("_t1" if slimq else "_gpu") if deterministic else ""))
+    threads = 1 if deterministic else 0
     graph = os.path.join(CACHE, f"hnsw_{'slimq' if slimq else 'slim'}_{tag}.graph")
     base = None
     if slimq:      # the raw rows are part of a hnsw_slimq index (exact rerank, setDataset)
@@ -108,16 +123,23 @@ def prepare_inputs(w: dict, n_query_batches: int, build_rank: bool, reference_bu
         tmp = graph + f".tmp{os.getpid()}"
         who = "engine host builder"
         if slimq:
-            capi.build_slimq_graph(base, tmp, M=w["M"], ef_construction=w["efc"], branching="4")
+            capi.build_slimq_graph(base, tmp, M=w["M"], ef_construction=w["efc"], branching="4", threads=threads)
         else:
             built = False
-            if reference_builder:
+            if deterministic:
+                gix = capi.Index.build_gpu(base, metric=w["metric"], M=w["M"], ef_construction=w["efc"], branching="4",
+                                           device=device)
+                gix.save(tmp)
+                gix.close()
+                built, who = True, "engine GPU builder (hs_build_slim_index_gpu, saved by hs_save_index)"
+            if reference_builder and not deterministic:
                 from oracle import refharness as rh
                 if rh.ref_slim_path() is not None:
                     rh.ref_slim_build(base, tmp, metric=w["metric"], M=w["M"], ef_construction=w["efc"], branching="4")
                     built, who = True, "reference builder (oracle/_ref)"
             if not built:
-                capi.build_slim_graph(base, tmp, metric=w["metric"], M=w["M"], ef_construction=w["efc"], branching="4")
+                capi.build_slim_graph(base, tmp, metric=w["metric"], M=w["M"], ef_construction=w["efc"], branching="4",
+                                      threads=threads)
         os.replace(tmp, graph)
         with open(graph + ".builder", "w") as f:
             f.write(who)
@@ -126,6 +148,41 @@ def prepare_inputs(w: dict, n_query_batches: int, build_rank: bool, reference_bu
     queries = [latent_gaussian(w["nq"], w["dim"], rank=w["rank"], seed=1, normalize=(w["metric"] == 1),
                                stream=1 + b) for b in range(n_query_batches)]
     return graph, base, queries
+
+
+def file_sha256(path: str) -> str:
+    import hashlib
+    h = hashlib.sha256()
+    with open(path, "rb") as f:
+        for blk in iter(lambda: f.read(1 << 24), b""):
+            h.update(blk)
+    return h.hexdigest()
+
+
+def index_sha256(ix) -> str:
+    """Digest of an index that lives in HBM only (GPU-built): of the file hs_save_index writes for it."""
+    import tempfile
+    with tempfile.TemporaryDirectory(prefix="hs_bench_") as td:
+        path = os.path.join(td, "index.graph")
+        ix.save(path)
+        return file_sha256(path)
+
+
+def dump_outputs(out_dir: str, labels: np.ndarray, dists: np.ndarray, inputs: dict) -> None:
+    """--dump-outputs: labels[nq,k] (ids, stored as float64: exact below 2**53), dists[nq,k] float32, and
+    inputs.json with digests of the index and the query batch the step searched: a comparison of two runs
+    refuses to compare outputs of different inputs."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "labels.npy"), labels.astype(np.float64))
+    np.save(os.path.join(out_dir, "distances.npy"), dists.astype(np.float32))
+    with open(os.path.join(out_dir, "inputs.json"), "w") as f:
+        json.dump(inputs, f, indent=1, sort_keys=True)
+    log(f"[bench] outputs of the last timed step ({labels.shape[0]} x {labels.shape[1]}) written to {out_dir}")
+
+
+def query_sha256(q: np.ndarray) -> str:
+    import hashlib
+    return hashlib.sha256(np.ascontiguousarray(q, dtype=np.float32).tobytes()).hexdigest()
 
 
 def graph_builder_of(graph: str) -> str:
@@ -322,10 +379,11 @@ def run_gpu(args, w):
     n_batches = min(8, args.warmup + args.steps)
     # rank 0 builds the graph (all host threads); the others wait, then read the cache
     if rank == 0:
-        graph, base, qbatches = prepare_inputs(w, n_batches, True)
+        graph, base, qbatches = prepare_inputs(w, n_batches, True, deterministic=bool(args.dump_outputs),
+                                               device=local_rank)
     barrier()
     if rank != 0:
-        graph, base, qbatches = prepare_inputs(w, n_batches, False)
+        graph, base, qbatches = prepare_inputs(w, n_batches, False, deterministic=bool(args.dump_outputs))
     # each rank takes its own batches (different streams) in the replicated/weak-scaling mode
     if distributed:
         from hnsw_slim_b200.synth import latent_gaussian
@@ -373,6 +431,10 @@ def run_gpu(args, w):
         stream.synchronize()
     barrier()
     ms_total = ev[0].elapsed_time(ev[-1])
+    if args.dump_outputs and rank == 0:      # before the sustained stream below reuses the buffers
+        dump_outputs(args.dump_outputs, d_lab.cpu().numpy().view(np.uint32), d_dist.cpu().numpy(),
+                     {"workload": args.workload, "k": k, "ef_search": w["ef"], "index_sha256": file_sha256(graph),
+                      "queries_sha256": query_sha256(qbatches[(args.warmup + args.steps - 1) % n_batches])})
     st = ix.stats()
     if distributed:
         t = torch.tensor([ms_total], device="cuda")
@@ -518,9 +580,9 @@ def run_gpu(args, w):
             ws["desc"] = ws["desc"].replace("in 8 ", f"in {ws['shards']} ")
         sargs = argparse.Namespace(**vars(args))
         sargs.ef = None
-        # a sharded step at 8 GPUs is ~0.3 ms and ranks depend on each other: K steps of it are dominated by
-        # the ranks' start-up skew, so the object times its own, larger number of steps (reported inside)
-        sargs.steps = max(args.steps, 200)
+        sargs.dump_outputs = None
+        # the object times --steps steps like the headline (before, at least 200): at 8 GPUs a window of a few
+        # ~0.3 ms steps is dominated by the ranks' start-up skew, so multi-GPU runs want a larger --steps
         try:
             sharded = measure_sharded(sargs, ws, rank, local_rank, world, dist if distributed else None)
         except Exception as e:          # the headline stands on its own; say why the object is missing
@@ -597,6 +659,10 @@ def run_gpu_bruteforce(args, w):
         stream.synchronize()
     barrier()
     ms_total = ev[0].elapsed_time(ev[1])
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_lab.cpu().numpy().view(np.uint32), d_dist.cpu().numpy(),
+                     {"workload": args.workload, "k": k, "base_sha256": query_sha256(base),
+                      "queries_sha256": query_sha256(qb[(args.warmup + args.steps - 1) % n_batches])})
     if distributed:
         t = torch.tensor([ms_total], device="cuda")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -738,6 +804,8 @@ def run_gpu_curve(args, w):
             e1.record(stream)
             stream.synchronize()
         ms = e0.elapsed_time(e1)
+        if args.dump_outputs:
+            last_out[ef] = (d_lab.cpu().numpy().view(np.uint32), d_dist.cpu().numpy())
         st = ix.stats()
         alg = (st["n_dist"] * 4 * info["dim_padded"] + st["n_hops"] * (8 + 4 * avg_deg0)) / steps
         gbs = alg / (ms / steps * 1e-3) / 1e9
@@ -746,6 +814,7 @@ def run_gpu_curve(args, w):
                 "alg_bytes": alg, "clocks": clocks.summary()}
 
     efs = [args.ef] if args.ef else [50, 100, 200, 400]
+    last_out = {}
     curve = [measure(ef, args.steps) for ef in efs]
     for c in curve:
         log(f"[bench] ef={c['ef_search']}: recall {c['recall_at_10']:.4f}, {c['qps']/1e6:.3f} M QPS, "
@@ -753,6 +822,10 @@ def run_gpu_curve(args, w):
     ok = [c for c in curve if c["recall_at_10"] >= 0.95]
     head = min(ok, key=lambda c: c["ef_search"]) if ok else max(curve, key=lambda c: c["recall_at_10"])
     ef = head["ef_search"]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *last_out[ef],
+                     {"workload": args.workload, "k": k, "ef_search": ef, "index_sha256": index_sha256(ix),
+                      "queries_sha256": query_sha256(qb[(args.warmup + args.steps - 1) % n_batches])})
 
     # end to end: pinned host batches in, pinned host rows out, three batches in flight (as the headline workload)
     ix.set_ef(ef)
@@ -1055,6 +1128,12 @@ def measure_sharded(args, w, rank, local_rank, world, dist):
         torch.cuda.synchronize()
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        digests = [file_sha256(paths[s]) if paths is not None else index_sha256(s_) for s, s_ in zip(mine, ix.shards)]
+        dump_outputs(args.dump_outputs, out[0].cpu().numpy().view(np.uint32), out[1].cpu().numpy(),
+                     {"workload": args.workload, "k": k, "ef_search_per_shard": ef, "shards": w["shards"],
+                      "rows_per_shard": w["n"] // w["shards"], "builder": builder, "shard_index_sha256": digests,
+                      "queries_sha256": query_sha256(qb[(args.warmup + args.steps - 1) % n_batches])})
     if rank == 0:
         log(f"[bench] sharded: {args.steps} steps in {ms:.2f} ms on rank 0")
     stats = [s_.stats() for s_ in ix.shards]          # counters of the K timed steps (before the sustained stream)
@@ -1250,7 +1329,12 @@ def main():
                     help="sharded workloads: NCCL all-gather, or the exchange fused into the traversal kernels")
     ap.add_argument("--no-sharded", action="store_true",
                     help="default workload: skip the embedded deep-sharded measurement (\"sharded\" object)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the labels and distances of the last timed step to DIR/labels.npy, DIR/distances.npy, "
+                         "digests of its inputs to DIR/inputs.json; host-built graphs are then built single-threaded")
     args = ap.parse_args()
+    if args.steps < 1:
+        raise SystemExit("bench.py: --steps must be at least 1")
     args.warmup = max(3, args.warmup) if args.impl == "ours" else max(1, args.warmup)
     w = dict(WORKLOADS[args.workload])
     if args.ef:
@@ -1263,6 +1347,8 @@ def main():
     if args.impl == "reference" and w.get("exact"):
         raise SystemExit("bench.py: --impl reference is defined for the graph-search workloads; the exact-kNN workload "
                          "times the reference's brute force inside its own line (cpu_baseline)")
+    if args.dump_outputs and args.impl == "reference":
+        raise SystemExit("bench.py: --dump-outputs is defined for the engine (--impl ours)")
     if args.impl == "reference":
         run_reference(args, w)
     elif w.get("exact"):

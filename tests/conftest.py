@@ -1,10 +1,11 @@
 """Shared fixtures.  `-m "not gpu"` runs on the CPU container (oracle, loader, ABI);
 `-m gpu` runs on a B200 and calls the CUDA path through the C ABI.
 
-Graphs are built with the REFERENCE builder (oracle/_ref, prebuilt here where /root/reference
-exists; the .so travels to the GPU box), single-threaded so that every box sees the same graph, and
-cached under a temp dir; where that library is
-unavailable the committed fixtures in tests/golden/ are used instead.
+Corpus graphs are built single-threaded, so that every machine sees the same graph, and cached
+under a temp dir: with the REFERENCE builder where the compiled reference (oracle/_ref) exists,
+with the engine's own host builder (hs_build_slim_graph) elsewhere.  Tests that run the reference
+itself skip without it; the golden tests check the small fixtures in tests/golden/, which hold
+outputs the reference produced on those fixtures only.
 """
 from __future__ import annotations
 
@@ -21,6 +22,7 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 from hnsw_slim_b200 import build as hs_build  # noqa: E402
+from hnsw_slim_b200 import capi as hs_capi  # noqa: E402
 from hnsw_slim_b200.synth import make_dataset  # noqa: E402
 from oracle import refharness as rh  # noqa: E402
 
@@ -64,21 +66,26 @@ needs_ref_hnsw = pytest.mark.skipif(rh.ref_hnsw_path() is None, reason="oracle/_
 
 
 class Corpus:
-    """A synthetic corpus + the reference-built .graph over it."""
+    """A synthetic corpus + a single-threaded .graph over it (reference builder if present, else the engine's)."""
 
     def __init__(self, n, nq, dim, metric=0, M=16, efc=200, rank=8, branching="4", seed=1, **prune):
         self.n, self.nq, self.dim, self.metric, self.M = n, nq, dim, metric, M
         self.base, self.queries = make_dataset(n, nq, dim, metric=metric, rank=rank, seed=seed)
-        # built SINGLE-THREADED: the reference's OpenMP build gives a different graph on every run, and a parity
+        # built SINGLE-THREADED: a multi-threaded build gives a different graph on every run, and a parity
         # suite must see the same graph (and the same distance ties) on every box
-        key = hashlib.sha1(repr(("1thread", n, dim, metric, M, efc, rank, branching, seed, sorted(prune.items()))).encode()
-                           ).hexdigest()[:16]
+        builder = "reference" if HAVE_REF else "engine"
+        key = hashlib.sha1(repr(("1thread", builder, n, dim, metric, M, efc, rank, branching, seed,
+                                 sorted(prune.items()))).encode()).hexdigest()[:16]
         os.makedirs(CACHE, exist_ok=True)
         self.graph = os.path.join(CACHE, f"slim_{key}.graph")
         if not os.path.exists(self.graph):
             tmp = self.graph + f".tmp{os.getpid()}"
-            rh.ref_slim_build(self.base, tmp, metric=metric, M=M, ef_construction=efc, branching=branching,
-                              threads=1, **prune)
+            if HAVE_REF:
+                rh.ref_slim_build(self.base, tmp, metric=metric, M=M, ef_construction=efc, branching=branching,
+                                  threads=1, **prune)
+            else:
+                hs_capi.build_slim_graph(self.base, tmp, metric=metric, M=M, ef_construction=efc, branching=branching,
+                                         threads=1, **prune)
             os.replace(tmp, self.graph)
 
 
@@ -88,8 +95,6 @@ _corpora: dict = {}
 def get_corpus(**kw) -> Corpus:
     key = repr(sorted(kw.items()))
     if key not in _corpora:
-        if not HAVE_REF:
-            pytest.skip("needs the reference builder (oracle/_ref)")
         _corpora[key] = Corpus(**kw)
     return _corpora[key]
 

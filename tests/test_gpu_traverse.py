@@ -83,13 +83,13 @@ def test_exact_ties_at_the_ef_boundary(tmp_path):
     Which of several equal-distance entries is trimmed / popped first is heap order in the reference and
     (lane, slot) order here.  This pins what that is allowed to change: the k returned DISTANCES (as a sorted
     multiset), never — only which of the identical copies carries a distance may differ, and with it the
-    counters."""
+    counters.  The graph comes from the engine's host builder, single-threaded, hence the same on every box."""
     rng = np.random.default_rng(123)
     distinct, copies, dim, nq, k = 2500, 3, 32, 400, 10
     d0, q = make_dataset(distinct, nq, dim, rank=8, seed=41)
     base = np.ascontiguousarray(np.repeat(d0, copies, axis=0)[rng.permutation(distinct * copies)])
     graph = str(tmp_path / "ties.graph")
-    rh.ref_slim_build(base, graph, M=8, ef_construction=60, threads=1)
+    capi.build_slim_graph(base, graph, M=8, ef_construction=60, threads=1)
     orc = rh.Oracle(graph, dim)
     ix = capi.Index(graph, dim)
     true_d = np.sort(((base[None, :, :] - q[:, None, :]) ** 2).sum(-1), axis=1)[:, :k]    # exact, tie-aware yardstick
@@ -108,7 +108,7 @@ def test_exact_ties_at_the_ef_boundary(tmp_path):
               f"identical counters {same_cnt.mean():.4f}, tie-aware recall gpu {hit(dist):.4f} oracle {hit(odist):.4f}")
         # the bound: the divergence may move WHICH copy is reported and how many hops it took, and in rare
         # cases reach one more / one fewer candidate — never more than 0.5 pp of recall, and at least 95 % of
-        # the rows carry bit-identical distances even in this all-ties corpus (measured: 97.5 % at ef=10)
+        # the rows carry bit-identical distances even in this all-ties corpus (measured on a B200: 99.75 % at ef=10)
         assert same_d.mean() >= 0.95, (ef, same_d.mean())
         assert abs(hit(dist) - hit(odist)) <= 0.005, (ef, hit(dist), hit(odist))
         # where the ids agree, the distances agree bitwise

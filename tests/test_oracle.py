@@ -222,15 +222,14 @@ def test_tie_events_are_reported():
         b = orc.search_ties(q, 10, ef, order=rh.ORDER_GPU, team=8)
         assert all(np.array_equal(x, y) for x, y in zip(a, b[:4]))
         assert int(b[4].sum()) == 0
-    if not rh.ref_slim_path():
-        pytest.skip("the all-ties corpus is built with the reference builder (oracle/_ref)")
+    from hnsw_slim_b200 import capi
     rng = np.random.default_rng(3)
     rows = rng.standard_normal((700, 16)).astype(np.float32)
     base = np.repeat(rows, 3, axis=0)                            # every vector three times, bit for bit
     queries = rng.standard_normal((60, 16)).astype(np.float32)
     with tempfile.TemporaryDirectory() as td:
         g = os.path.join(td, "ties.graph")
-        rh.ref_slim_build(base, g, M=8, ef_construction=60, threads=1)
+        capi.build_slim_graph(base, g, M=8, ef_construction=60, threads=1)   # single-threaded: the same graph on every box
         orc = rh.Oracle(g, 16)
         a = orc.search(queries, 10, 12, order=rh.ORDER_GPU, team=8)
         b = orc.search_ties(queries, 10, 12, order=rh.ORDER_GPU, team=8)
@@ -257,16 +256,16 @@ def test_pool_emulator_equals_the_reference_semantics(name, metric):
         orc.search_pool(q, 10, 300)                              # register pools only
 
 
-@needs_ref
 def test_pool_emulator_on_a_live_corpus():
     """The same on a 20k x 128 corpus, plus the all-ties corpus where the two algorithms are ALLOWED to part:
     the emulator must still return a valid answer (sorted, distinct ids) with recall equal within 0.5 pp."""
     import tempfile
+    from hnsw_slim_b200 import capi
     from hnsw_slim_b200.synth import make_dataset
     base, q = make_dataset(20000, 300, 128, rank=14, seed=2)
     with tempfile.TemporaryDirectory() as td:
         g = os.path.join(td, "g.graph")
-        rh.ref_slim_build(base, g, M=16, ef_construction=100, threads=1)
+        capi.build_slim_graph(base, g, M=16, ef_construction=100, threads=1)     # single-threaded: the same graph on every box
         orc = rh.Oracle(g, 128)
         for ef in (50, 100, 200):
             lab, dist, nd, nh, nt = orc.search_ties(q, 10, ef, order=rh.ORDER_GPU, team=8)
@@ -279,7 +278,7 @@ def test_pool_emulator_on_a_live_corpus():
         tb = np.repeat(rows, 3, axis=0)
         tq = rng.standard_normal((60, 16)).astype(np.float32)
         g2 = os.path.join(td, "ties.graph")
-        rh.ref_slim_build(tb, g2, M=8, ef_construction=60, threads=1)
+        capi.build_slim_graph(tb, g2, M=8, ef_construction=60, threads=1)
         o2 = rh.Oracle(g2, 16)
         for ef in (12, 24, 40):
             lab, dist, *_ = o2.search_ties(tq, 10, ef, order=rh.ORDER_GPU, team=8)
