@@ -1149,7 +1149,13 @@ int hs_bruteforce_knn(const float *base, size_t n, size_t dim, const float *quer
   }
   int rc = select_device(device);
   if (rc != HS_OK) return rc;
-  if (nq == 0 || n == 0) return HS_OK;
+  if (nq == 0) return HS_OK;
+  // checked before the n == 0 return below: with no base rows there is nothing to write k rows from
+  if (k > n) {
+    set_error("bruteforce: k > n (bruteforce.h:107 asserts k <= cur_element_count)");
+    return HS_ERR_ARG;
+  }
+  if (n == 0) return HS_OK;
   float *d_base = nullptr, *d_q = nullptr, *d_dist = nullptr;
   uint32_t *d_lab = nullptr;
   size_t bytes = 0;

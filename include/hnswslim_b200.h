@@ -356,7 +356,7 @@ int hs_reset_stats(hs_index *);
  * BruteforceSearch<float>::searchKnn per query (bruteforce.h:106-135): exact kNN of
  * nq queries over n base rows (label of row i = i).  Row order: NEAREST first,
  * ties -> smaller label (the reference writes farthest-first; reverse to compare).
- * Host buffers; dists_out may be NULL. */
+ * Host buffers; dists_out may be NULL.  k > n is HS_ERR_ARG whenever nq > 0 (also for n == 0). */
 int hs_bruteforce_knn(const float *base, size_t n, size_t dim, const float *queries, size_t nq,
                       size_t k, int metric, int device, uint32_t *labels_out, float *dists_out);
 
