@@ -31,7 +31,7 @@ EXPORTS = [
     "hs_shardgroup_free", "hs_build_slim_index_gpu", "hs_save_index", "hs_build_slimq_index_gpu",
     "hs_load_reserve", "hs_patch_apply", "hs_debug_patch",
     "hs_service_create", "hs_service_query", "hs_service_set_ef", "hs_service_patch", "hs_service_get_stats",
-    "hs_service_free", "hs_debug_service_create", "hs_set_tuning",
+    "hs_service_free", "hs_debug_service_create", "hs_set_tuning", "hs_debug_convert_gpu", "hs_debug_slimq_payload",
 ]
 HS_PATCH_INLINE_ROWS = 1
 
@@ -181,6 +181,8 @@ def lib():
         L.hs_get_query_tconst.argtypes = [vp, C.POINTER(C.c_double)]
         L.hs_set_query_tconst.argtypes = [vp, C.c_double]
         L.hs_slimq_prepare.argtypes = [vp, vp, sz, vp, vp, vp, vp]
+        L.hs_debug_convert_gpu.argtypes = [C.c_char_p, sz, i32, C.POINTER(BuildParams), i32, C.POINTER(vp)]
+        L.hs_debug_slimq_payload.argtypes = [vp, vp, vp, vp]
         for name in EXPORTS:
             if name not in ("hs_last_error", "hs_free", "hs_debug_free", "hs_build_params_default", "hs_exchange_free",
                             "hs_shardgroup_free", "hs_service_free",
@@ -280,9 +282,39 @@ class Index:
         self.dim = dim
         return self
 
+    @classmethod
+    def convert_gpu(cls, hnsw_path: str, dim: int, *, metric: int = HS_METRIC_L2, device: int = 0,
+                    **prune) -> "Index":
+        """hs_debug_convert_gpu: the device builder's convertFromHNSW (phase 2) over the lists of an
+        hs_build_hnsw_graph file; `prune` sets threshold_level, top_degree_percent, top_M0, low_m0, top_M, low_m."""
+        self = cls.__new__(cls)
+        self._h = C.c_void_p()
+        p = BuildParams()
+        lib().hs_build_params_default(C.byref(p))
+        for k_, v in prune.items():
+            setattr(p, k_, v)
+        _check(lib().hs_debug_convert_gpu(hnsw_path.encode(), dim, metric, C.byref(p), device, C.byref(self._h)))
+        self.dim = dim
+        return self
+
     def save(self, path: str) -> None:
         """hs_save_index: the reference's saveIndex format (slim.h:717-751)."""
         _check(lib().hs_save_index(self._h, path.encode()))
+
+    def slimq_payload(self) -> dict:
+        """hs_debug_slimq_payload (hnsw_slimq): per node codes[n, words] (MSB-first u64 words), f_add[n],
+        f_rescale[n], cluster[n]; the rotated centroids[num_cluster, padded_dim] and the rotator flip bytes."""
+        info = self.info()
+        n, pd, nc = info["n"], info["padded_dim_q"], info["num_cluster"]
+        words = pd // 64
+        rec = np.zeros((n, words + 2), np.uint64)
+        cent = np.zeros((nc, pd), np.float32)
+        flip = np.zeros(4 * pd // 8, np.uint8)
+        _check(lib().hs_debug_slimq_payload(self._h, rec.ctypes.data, cent.ctypes.data, flip.ctypes.data))
+        fac = rec[:, words].copy().view(np.float32).reshape(n, 2)
+        return {"codes": rec[:, :words].copy(), "f_add": fac[:, 0].copy(), "f_rescale": fac[:, 1].copy(),
+                "cluster": (rec[:, words + 1] & np.uint64(0xFFFFFFFF)).astype(np.uint32),
+                "centroids": cent, "flip": flip}
 
     def close(self) -> None:
         if getattr(self, "_h", None):

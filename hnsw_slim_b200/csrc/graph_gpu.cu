@@ -1138,6 +1138,42 @@ int convert_gpu(const float4 *d_vec, uint32_t row_chunks, int metric, const GpuH
 // ---- entry points used by hs_api.cu ----
 namespace {
 
+// phase 2 and the hand-over: convertFromHNSW over g's lists (adj0 / up[l], strides stride0 / ustride), then the
+// vector store, the slots and the slim lists move into `dg`
+int convert_into_device_graph(DevBuf &vec, size_t n, size_t dim, size_t dim_padded, int metric, GpuHnsw &g,
+                              const hs_build_params *bp, cudaStream_t st, DeviceGraph *dg) {
+  const uint32_t row_chunks = (uint32_t)(dim_padded / 4);
+  ConvertParams cp{bp->threshold_level, bp->top_degree_percent0, bp->top_degree_percent, (uint32_t)bp->top_M0,
+                   (uint32_t)bp->low_m0, (uint32_t)bp->top_M, (uint32_t)bp->low_m};
+  GpuSlim s;
+  const uint32_t *hup[kMaxLevels] = {};
+  for (int l = 1; l <= g.maxlevel; ++l) hup[l] = g.up[l].as<uint32_t>();
+  const int rc = convert_gpu(vec.as<float4>(), row_chunks, metric, g, g.adj0.as<uint32_t>(), g.stride0, hup, g.ustride, cp, st, &s);
+  if (rc != HS_OK) return rc;
+  dg->n = n;
+  dg->dim = dim;
+  dg->dim_padded = dim_padded;
+  dg->metric = metric;
+  dg->M = g.M;
+  dg->maxM = g.maxM;
+  dg->maxM0 = g.maxM0;
+  dg->ef_construction = g.efc;
+  dg->maxlevel = g.maxlevel;
+  dg->threshold_level = bp->threshold_level;
+  dg->enterpoint = g.ep;
+  dg->deg0_stride = s.deg0_stride;
+  dg->max_deg0 = s.max_deg0;
+  dg->upper_stride = s.upper_stride;
+  dg->n_upper = g.n_upper;
+  dg->sum_deg0 = s.sum_deg0;
+  for (int l = 0; l <= g.maxlevel; ++l) dg->level_count[l] = g.level_count[l];
+  dg->d_vec = static_cast<float *>(vec.release());
+  dg->d_adj0 = static_cast<uint32_t *>(s.adj0.release());
+  dg->d_upper_slot = static_cast<int32_t *>(g.slot.release());
+  for (int l = 1; l <= g.maxlevel; ++l) dg->d_upper_adj[l] = static_cast<uint32_t *>(s.up[l].release());
+  return HS_OK;
+}
+
 // rows -> HNSW -> HNSW-Slim lists, all on the device; fills `dg` (ownership of the arrays moves to it)
 int build_slim_device_graph(const float *base, size_t n, size_t dim, int metric, const hs_build_params *bp,
                             double branching, int device, cudaStream_t st, DeviceGraph *dg) {
@@ -1166,34 +1202,39 @@ int build_slim_device_graph(const float *base, size_t n, size_t dim, int metric,
   GpuHnsw g;
   rc = build_hnsw_gpu(vec.as<float4>(), row_chunks, n, metric, bp->M, bp->ef_construction, branching, bp->seed, st, &g);
   if (rc != HS_OK) return rc;
-  ConvertParams cp{bp->threshold_level, bp->top_degree_percent0, bp->top_degree_percent, (uint32_t)bp->top_M0,
-                   (uint32_t)bp->low_m0, (uint32_t)bp->top_M, (uint32_t)bp->low_m};
-  GpuSlim s;
-  const uint32_t *hup[kMaxLevels] = {};
-  for (int l = 1; l <= g.maxlevel; ++l) hup[l] = g.up[l].as<uint32_t>();
-  rc = convert_gpu(vec.as<float4>(), row_chunks, metric, g, g.adj0.as<uint32_t>(), g.stride0, hup, g.ustride, cp, st, &s);
-  if (rc != HS_OK) return rc;
-  dg->n = n;
-  dg->dim = dim;
-  dg->dim_padded = dim_padded;
-  dg->metric = metric;
-  dg->M = g.M;
-  dg->maxM = g.maxM;
-  dg->maxM0 = g.maxM0;
-  dg->ef_construction = g.efc;
-  dg->maxlevel = g.maxlevel;
-  dg->threshold_level = bp->threshold_level;
-  dg->enterpoint = g.ep;
-  dg->deg0_stride = s.deg0_stride;
-  dg->max_deg0 = s.max_deg0;
-  dg->upper_stride = s.upper_stride;
-  dg->n_upper = g.n_upper;
-  dg->sum_deg0 = s.sum_deg0;
-  for (int l = 0; l <= g.maxlevel; ++l) dg->level_count[l] = g.level_count[l];
-  dg->d_vec = static_cast<float *>(vec.release());
-  dg->d_adj0 = static_cast<uint32_t *>(s.adj0.release());
-  dg->d_upper_slot = static_cast<int32_t *>(g.slot.release());
-  for (int l = 1; l <= g.maxlevel; ++l) dg->d_upper_adj[l] = static_cast<uint32_t *>(s.up[l].release());
+  return convert_into_device_graph(vec, n, dim, dim_padded, metric, g, bp, st, dg);
+}
+
+// The un-pruned lists of an hs_build_hnsw_graph file as a phase-1 result: the file's levels, entry point and
+// M / maxM / maxM0, the loader's slot order (= assign_slots'), and rows re-strided to the widths the phase-2
+// kernels read (round_up(maxM0 | maxM, 32) ids, kInvalid-padded).
+int device_hnsw_from_file(const HostGraph &h, cudaStream_t st, GpuHnsw *out) {
+  GpuHnsw &g = *out;
+  g.M = (uint32_t)h.M;
+  g.maxM = (uint32_t)h.maxM;
+  g.maxM0 = (uint32_t)h.maxM0;
+  g.efc = (uint32_t)h.ef_construction;
+  g.levels = h.levels;
+  g.maxlevel = h.maxlevel;
+  int rc;
+  if ((rc = assign_slots(g)) != HS_OK) return rc;
+  g.ep = h.enterpoint;
+  g.stride0 = round_up(g.maxM0, 32);
+  g.ustride = round_up(g.maxM, 32);
+  auto upload_rows = [&](const std::vector<uint32_t> &src, uint32_t sstride, size_t rows, uint32_t dstride,
+                         DevBuf &dst) -> int {
+    std::vector<uint32_t> w(rows * dstride, kInvalid);
+    const uint32_t c = std::min(sstride, dstride);
+    for (size_t r = 0; r < rows; ++r) std::memcpy(&w[r * dstride], &src[r * sstride], 4 * (size_t)c);
+    int rc2;
+    if ((rc2 = dst.alloc(w.size() * 4)) != HS_OK) return rc2;
+    GB_CUDA(cudaMemcpyAsync(dst.p, w.data(), w.size() * 4, cudaMemcpyHostToDevice, st));
+    GB_CUDA(cudaStreamSynchronize(st));
+    return HS_OK;
+  };
+  if ((rc = upload_rows(h.adj0, h.deg0_stride, h.n, g.stride0, g.adj0)) != HS_OK) return rc;
+  for (int l = 1; l <= g.maxlevel; ++l)
+    if ((rc = upload_rows(h.upper_adj[l], h.upper_stride, g.level_count[l], g.ustride, g.up[l])) != HS_OK) return rc;
   return HS_OK;
 }
 
@@ -1234,6 +1275,40 @@ int gpu_build_slim_index(const float *base, size_t n, size_t dim, int metric, co
   std::vector<uint32_t> lab(n);
   for (size_t i = 0; i < n; ++i) lab[i] = labels ? (uint32_t)labels[i] : (uint32_t)i;     // truncated as slim.h:2129
   dg.h_labels = lab.data();
+  return adopt_device_graph(dg, device, out_ix);
+}
+
+// phase 2 of gpu_build_slim_index over the lists of an hs_build_hnsw_graph file (hs_debug_convert_gpu)
+int gpu_debug_convert(const char *hnsw_graph_path, size_t dim, int metric, const hs_build_params *bp, int device,
+                      hs_index **out_ix) {
+  int rc = select_device(device);
+  if (rc != HS_OK) return rc;
+  HostGraph h;
+  {
+    std::vector<uint8_t> bytes;
+    if ((rc = read_file(hnsw_graph_path, &bytes)) != HS_OK) return rc;
+    if ((rc = parse_graph(bytes.data(), bytes.size(), HS_KIND_HNSW, dim, &h)) != HS_OK) return rc;
+  }
+  if (h.n == 0) {
+    set_error("hs_debug_convert_gpu: the index is empty");
+    return HS_ERR_ARG;
+  }
+  cudaStream_t st = nullptr;
+  GB_CUDA(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
+  StreamGuard guard{st};
+  DeviceGraph dg;
+  {
+    DevBuf vec;
+    GpuHnsw g;
+    if ((rc = vec.alloc(h.vec.size() * 4)) != HS_OK) return rc;
+    GB_CUDA(cudaMemcpyAsync(vec.p, h.vec.data(), h.vec.size() * 4, cudaMemcpyHostToDevice, st));
+    if ((rc = device_hnsw_from_file(h, st, &g)) != HS_OK ||
+        (rc = convert_into_device_graph(vec, h.n, dim, h.dim_padded, metric, g, bp, st, &dg)) != HS_OK) {
+      free_device_graph(dg);
+      return rc;
+    }
+  }
+  dg.h_labels = h.labels.data();
   return adopt_device_graph(dg, device, out_ix);
 }
 

@@ -1350,6 +1350,38 @@ int hs_build_slimq_index_gpu(const float *base, size_t n, size_t dim, const hs_b
   });
 }
 
+int hs_debug_convert_gpu(const char *hnsw_graph_path, size_t dim, int metric, const hs_build_params *p, int device,
+                         hs_index **out) {
+  if (!out) {
+    set_error("null argument");
+    return HS_ERR_ARG;
+  }
+  *out = nullptr;
+  if (!hnsw_graph_path || !p || dim == 0 || (metric != HS_METRIC_L2 && metric != HS_METRIC_IP)) {
+    set_error("hs_debug_convert_gpu: bad argument");
+    return HS_ERR_ARG;
+  }
+  return guarded("hs_debug_convert_gpu", [&] { return gpu_debug_convert(hnsw_graph_path, dim, metric, p, device, out); });
+}
+
+int hs_debug_slimq_payload(const hs_index *ix, uint64_t *records, float *rotated_centroids, uint8_t *flip) {
+  if (!ix) {
+    set_error("null argument");
+    return HS_ERR_ARG;
+  }
+  if (ix->info.kind != HS_KIND_SLIMQ) {
+    set_error("hs_debug_slimq_payload: not an hnsw_slimq index");
+    return HS_ERR_ARG;
+  }
+  const hs_index_info &I = ix->info;
+  HS_CUDA(cudaSetDevice(ix->device));
+  if (records) HS_CUDA(cudaMemcpy(records, ix->d_qrec, I.n * (I.padded_dim_q / 64 + 2) * 8, cudaMemcpyDeviceToHost));
+  if (rotated_centroids)
+    HS_CUDA(cudaMemcpy(rotated_centroids, ix->d_centroids, I.num_cluster * I.padded_dim_q * 4, cudaMemcpyDeviceToHost));
+  if (flip) HS_CUDA(cudaMemcpy(flip, ix->d_flip, 4 * I.padded_dim_q / 8, cudaMemcpyDeviceToHost));
+  return HS_OK;
+}
+
 // saveIndex (slim.h:717-751) of an HBM-resident hnsw_slim index: header, element records
 // [int32 level][uint32 total][uint64 label][8 stale pointer bytes][float vec[dim]], then per node
 // uint32 blob size + [uint16 offsets[level]][uint32 ids[total]].

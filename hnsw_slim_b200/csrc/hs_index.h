@@ -124,5 +124,7 @@ int gpu_build_slim_index(const float *base, size_t n, size_t dim, int metric, co
 int gpu_build_slimq_index(const float *base, size_t n, size_t dim, const hs_build_params *bp, double branching,
                           const float *centroids, size_t num_cluster, const uint64_t *labels, int device,
                           hs_index **out);
+int gpu_debug_convert(const char *hnsw_graph_path, size_t dim, int metric, const hs_build_params *bp, int device,
+                      hs_index **out);
 
 }  // namespace hs

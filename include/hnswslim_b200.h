@@ -467,6 +467,20 @@ int hs_debug_node(const hs_host_graph *, uint32_t node, int *level, uint32_t *la
  * are the code the device path runs; the level-0 rows and vectors are written to the host arrays instead. */
 int hs_debug_patch(hs_host_graph *, const void *patch, size_t patch_bytes, unsigned flags, const float *rows,
                    const uint64_t *row_labels, size_t n_rows, hs_patch_info *info_out);
+/* Phase 2 of hs_build_slim_index_gpu alone: the same device code (convertFromHNSW, slim.h:867-1108) run on the
+ * un-pruned lists of an hs_build_hnsw_graph file instead of a device-built HNSW graph, so that its lists can be
+ * compared one by one with hs_build_slim_graph's conversion of the same file.  Vectors, levels, labels, entry point
+ * and M / maxM / maxM0 come from the file; threshold_level, top_degree_percent, top_M0, low_m0, top_M and low_m
+ * from `p`.  The result is an hnsw_slim index (hs_save_index writes it).  Needs maxM0 <= 64 and pruning
+ * parameters <= 64 (HS_ERR_UNSUPPORTED otherwise, as for the builder). */
+int hs_debug_convert_gpu(const char *hnsw_graph_path, size_t dim, int metric, const hs_build_params *p, int device,
+                         hs_index **out);
+/* hnsw_slimq only, inspection: the per-node payload as the traversal kernel reads it, for an index built on the
+ * device or loaded with hs_load.  records: n x (padded_dim/64 + 2) 8-byte words, per node the code words (bit
+ * 63 - j of word w = sign of dimension 64w + j, the file's MSB-first order), then (f_add, f_rescale) as two floats,
+ * then (cluster id, 0) as two uint32; rotated_centroids: num_cluster x padded_dim; flip: 4 * padded_dim / 8
+ * rotator sign bytes.  Any output may be NULL. */
+int hs_debug_slimq_payload(const hs_index *, uint64_t *records, float *rotated_centroids, uint8_t *flip);
 
 const char *hs_last_error(void);
 int hs_abi_version(void);
