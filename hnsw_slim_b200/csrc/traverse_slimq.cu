@@ -192,7 +192,12 @@ __device__ __forceinline__ void prepare_query(const TraverseQParams &p, const fl
     }
   }
   const float norm_quan = __fsqrt_rn(warp_sum_f(s_uu));
-  const float cosv = __fdiv_rn(warp_sum_f(s_ru), __fmul_rn(norm_data, norm_quan));
+  // norm_data == 0 (an all-zero query, or one whose squares underflow): the reference computes cosv = 0 / 0, so
+  // delta, vl and every estimate are NaN, and a NaN key, f2ord(0x7fffffff) == 0xffffffff, is the pool's
+  // "expanded / empty" marker: the base-layer search would stop at once and return one result and padding.
+  // This departs from the reference on purpose and takes the limit cosv = 0 (delta = vl = 0): the estimate is
+  // then f_add + ||c||^2, RaBitQ's estimate of ||x||^2, which is the distance to a zero query.  The oracle agrees.
+  const float cosv = norm_data > 0.f ? __fdiv_rn(warp_sum_f(s_ru), __fmul_rn(norm_data, norm_quan)) : 0.f;
   delta = __fmul_rn(__fdiv_rn(norm_data, norm_quan), cosv);            // :567
   vl = __fmul_rn(delta, -7.5f);                                         // :574
   k1xsumq = __fmul_rn(sumq, -0.5f);                                     // query.hpp:133,138

@@ -326,7 +326,11 @@ void hsoq_quantize_query(const hsoq_index *ix, const float *rq, uint64_t *planes
     tmp[i] = (float)u;
   }
   const float norm_quan = sqrtf(warp_dot(ucb, ucb, pd));      /* :562 */
-  const float cosv = warp_dot(rq, ucb, pd) / (norm_data * norm_quan);   /* :563-564 */
+  /* :563-564.  norm_data == 0 (zero query, or squares that underflow): the reference divides 0 by 0 and every
+   * estimate is NaN, which qb_is_full never rejects, so its search walks the whole reachable graph.  We depart
+   * from it on purpose: cosv = 0, so delta = vl = 0 and the estimate is f_add + |c|^2, the RaBitQ estimate of
+   * |x|^2 (traverse_slimq.cu does the same). */
+  const float cosv = norm_data > 0.f ? warp_dot(rq, ucb, pd) / (norm_data * norm_quan) : 0.f;
   const float delta = norm_data / norm_quan * cosv;           /* :567 (RECONSTRUCTION) */
   scal[0] = delta;
   scal[1] = delta * -7.5f;                                    /* :574 */
