@@ -298,7 +298,9 @@ class Index:
         return self
 
     def save(self, path: str) -> None:
-        """hs_save_index: the reference's saveIndex format (slim.h:717-751)."""
+        """hs_save_index: the reference's saveIndex format, hnsw_slim (slim.h:717-751) or hnsw_slimq
+        (slimq.h:1161-1216).  An hnsw_slimq file is written with zero ex-code blocks and holds no raw rows: open it
+        again with the same rows, in the same order, as raw_base (for a GPU-built index, the builder's input)."""
         _check(lib().hs_save_index(self._h, path.encode()))
 
     def slimq_payload(self) -> dict:

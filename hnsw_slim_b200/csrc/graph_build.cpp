@@ -719,18 +719,15 @@ int build_slimq_graph(const float *base, size_t n, size_t dim, size_t M, size_t 
   std::vector<float> rcent(num_cluster * pd);
   for (size_t c = 0; c < num_cluster; ++c) host_rotate(centroids + c * dim, dim, pd, td, flip.data(), &rcent[c * pd]);
 
-  // record layout (slimq.h:1498-1505): [level][total][label][ptr][cluster @24][bin @28][ex]
-  const size_t ex_bits = 3;
-  const uint64_t size_bin = pd / 8 + 12, size_ex = pd * ex_bits / 8 + 8;     // data_layout.hpp
-  const uint64_t off_bin = 28, off_ex = off_bin + size_bin, rec = off_ex + size_ex;
-  std::vector<uint8_t> elements(n * rec, 0);
+  // one_bit_code_with_factor (rabitq_impl.hpp:76-135, L2 metric) per node, in double
+  std::vector<uint64_t> codes(n * words, 0);
+  std::vector<float> fac(3 * n);                                // f_add, f_rescale, f_error
   parallel_for(0, n, threads, [&](size_t i, int) {
-    std::vector<float> rot(pd), res(pd);
+    std::vector<float> rot(pd);
     host_rotate(base + i * dim, dim, pd, td, flip.data(), rot.data());
     const float *cen = &rcent[(size_t)cluster_ids[i] * pd];
-    // one_bit_code_with_factor, rabitq_impl.hpp:76-135 (L2 metric), in double
     double l2 = 0, ip_resi = 0, ip_cent = 0;
-    std::vector<uint64_t> code(words, 0);
+    uint64_t *code = &codes[i * words];
     for (size_t d = 0; d < pd; ++d) {
       const float r = rot[d] - cen[d];
       const int bit = r > 0.f ? 1 : 0;
@@ -744,53 +741,103 @@ int build_slimq_graph(const float *base, size_t n, size_t dim, size_t M, size_t 
     const double l2n = std::sqrt(l2);
     const double tmp_err =
         l2n * 1.9 * std::sqrt(std::max(0.0, (l2 * ((double)pd * 0.25) / (ip_resi * ip_resi) - 1.0) / (double)(pd - 1)));
-    const float f_add = (float)(l2 + 2 * l2 * ip_cent / ip_resi);
-    const float f_rescale = (float)(-2 * l2 / ip_resi);
-    const float f_error = (float)(2 * tmp_err);
-    uint8_t *e = &elements[i * rec];
-    uint32_t total = 0;
-    for (auto &l : P.nbr[i]) total += (uint32_t)l.size();
-    const int32_t lv = h.level[i];
-    const uint64_t label = labels ? labels[i] : (uint64_t)i;
-    std::memcpy(e, &lv, 4);
-    std::memcpy(e + 4, &total, 4);
-    std::memcpy(e + 8, &label, 8);
-    std::memcpy(e + 24, &cluster_ids[i], 4);
-    std::memcpy(e + off_bin, code.data(), 8 * words);
-    std::memcpy(e + off_bin + 8 * words, &f_add, 4);
-    std::memcpy(e + off_bin + 8 * words + 4, &f_rescale, 4);
-    std::memcpy(e + off_bin + 8 * words + 8, &f_error, 4);
-    // the ex-code block (3 extra bits per dimension) is left zero: the search path never reads
-    // it (SURVEY.md App. A: only get_bin_est is called, slimq.h:737-738)
+    fac[3 * i] = (float)(l2 + 2 * l2 * ip_cent / ip_resi);
+    fac[3 * i + 1] = (float)(-2 * l2 / ip_resi);
+    fac[3 * i + 2] = (float)(2 * tmp_err);
   });
 
-  FILE *f = std::fopen(out_path, "wb");
+  SlimqHead head;
+  head.n = n;
+  head.maxlevel = P.maxlevel;
+  head.threshold_level = threshold_level;
+  head.enterpoint = h.enter.load();
+  head.maxM = h.maxM;
+  head.maxM0 = h.maxM0;
+  head.M = h.M;
+  head.ef_construction = h.efc;
+  head.num_cluster = num_cluster;
+  head.dim = dim;
+  head.padded_dim = pd;
+  head.ex_bits = 3;
+  head.size_ex = pd * 3 / 8 + 8;                                // data_layout.hpp
+  head.centroids = rcent.data();
+  head.flip = flip.data();
+  return write_slimq_file(
+      out_path, head,
+      [&](size_t i0, size_t cnt, SlimqNode *out) -> int {
+        for (size_t j = 0; j < cnt; ++j) {
+          const size_t i = i0 + j;
+          SlimqNode &nd = out[j];
+          nd.level = h.level[i];
+          nd.total = 0;
+          for (auto &l : P.nbr[i]) nd.total += (uint32_t)l.size();
+          nd.label = labels ? labels[i] : (uint64_t)i;
+          nd.cluster = cluster_ids[i];
+          nd.code = &codes[i * words];
+          nd.f_add = fac[3 * i];
+          nd.f_rescale = fac[3 * i + 1];
+          nd.f_error = fac[3 * i + 2];
+        }
+        return HS_OK;
+      },
+      [&](FILE *f) { return write_blobs(f, P); });
+}
+
+int write_slimq_file(const char *path, const SlimqHead &h,
+                     const std::function<int(size_t i0, size_t cnt, SlimqNode *out)> &nodes,
+                     const std::function<bool(FILE *f)> &blobs) {
+  // record layout (slimq.h:1498-1505): [level][total][label][ptr][cluster @24][bin @28][ex]
+  const size_t words = h.padded_dim / 64;
+  const uint64_t size_bin = h.padded_dim / 8 + 12;             // data_layout.hpp
+  const uint64_t off_bin = 28, off_ex = off_bin + size_bin, rec = off_ex + h.size_ex;
+  FILE *f = std::fopen(path, "wb");
   if (!f) {
-    set_error(std::string("cannot open ") + out_path + " for writing");
+    set_error(std::string("cannot open ") + path + " for writing");
     return HS_ERR_IO;
   }
   auto put = [&](const void *p, size_t sz) { return std::fwrite(p, 1, sz, f) == sz; };
   bool ok = true;
-  const uint64_t hdr[6] = {n, rec, 8, 4, off_bin /* offsetData_ = offset_bin_data_, slimq.h:1503 */, 16};
+  const uint64_t hdr[6] = {h.n, rec, 8, 4, off_bin /* offsetData_ = offset_bin_data_, slimq.h:1503 */, 16};
   ok &= put(hdr, sizeof hdr);
-  const int32_t ml = P.maxlevel, thr = threshold_level;
-  const uint32_t ep = h.enter.load();
-  ok &= put(&ml, 4) && put(&thr, 4) && put(&ep, 4);
-  const uint64_t ms[4] = {h.maxM, h.maxM0, h.M, h.efc};
+  ok &= put(&h.maxlevel, 4) && put(&h.threshold_level, 4) && put(&h.enterpoint, 4);
+  const uint64_t ms[4] = {h.maxM, h.maxM0, h.M, h.ef_construction};
   ok &= put(ms, sizeof ms);
   const uint8_t has_deleted = 0;
   ok &= put(&has_deleted, 1);
-  const uint64_t meta[9] = {num_cluster, dim, pd, 24, off_bin, off_ex, size_bin, size_ex, ex_bits};
+  const uint64_t meta[9] = {h.num_cluster, h.dim, h.padded_dim, 24, off_bin, off_ex, size_bin, h.size_ex, h.ex_bits};
   ok &= put(meta, sizeof meta);
   const uint8_t metric_type = 0;   // rabitqlib::METRIC_L2
   ok &= put(&metric_type, 1);
-  ok &= put(rcent.data(), rcent.size() * 4);
-  ok &= put(flip.data(), flip.size());
-  ok &= put(elements.data(), elements.size());
-  ok = ok && write_blobs(f, P);
+  ok &= put(h.centroids, h.num_cluster * h.padded_dim * 4);
+  ok &= put(h.flip, 4 * h.padded_dim / 8);
+  const size_t slab = std::max<size_t>(1, (64u << 20) / rec);
+  std::vector<SlimqNode> nd(std::min<size_t>(slab, h.n));
+  std::vector<uint8_t> buf(nd.size() * rec);
+  for (size_t i0 = 0; i0 < h.n && ok; i0 += slab) {
+    const size_t cnt = std::min<size_t>(slab, h.n - i0);
+    const int rc = nodes(i0, cnt, nd.data());
+    if (rc != HS_OK) {
+      std::fclose(f);
+      return rc;
+    }
+    std::fill(buf.begin(), buf.end(), 0);
+    for (size_t j = 0; j < cnt; ++j) {
+      uint8_t *e = &buf[j * rec];
+      std::memcpy(e, &nd[j].level, 4);
+      std::memcpy(e + 4, &nd[j].total, 4);
+      std::memcpy(e + 8, &nd[j].label, 8);
+      std::memcpy(e + 24, &nd[j].cluster, 4);
+      std::memcpy(e + off_bin, nd[j].code, 8 * words);
+      std::memcpy(e + off_bin + 8 * words, &nd[j].f_add, 4);
+      std::memcpy(e + off_bin + 8 * words + 4, &nd[j].f_rescale, 4);
+      std::memcpy(e + off_bin + 8 * words + 8, &nd[j].f_error, 4);
+    }
+    ok &= put(buf.data(), cnt * rec);
+  }
+  ok = ok && blobs(f);
   ok &= std::fclose(f) == 0;
   if (!ok) {
-    set_error(std::string("write error on ") + out_path);
+    set_error(std::string("write error on ") + path);
     return HS_ERR_IO;
   }
   return HS_OK;

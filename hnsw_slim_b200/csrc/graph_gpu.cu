@@ -616,6 +616,7 @@ struct PayloadParams {
   const uint8_t *flip;            // 4 * pd / 8
   float fac;                      // 1 / sqrt(td)
   uint2 *qrec;                    // n x (words + 2)
+  float *f_error;                 // n (the file's third factor; the search does not read it)
 };
 
 __global__ void __launch_bounds__(128) slimq_payload_kernel(const __grid_constant__ PayloadParams p) {
@@ -714,8 +715,11 @@ __global__ void __launch_bounds__(128) slimq_payload_kernel(const __grid_constan
     if (ip_resi == 0) ip_resi = __longlong_as_double(0x7ff0000000000000ll);
     const float f_add = (float)(l2 + 2 * l2 * ip_cent / ip_resi);
     const float f_rescale = (float)(-2 * l2 / ip_resi);
+    const double tmp_err =
+        sqrt(l2) * 1.9 * sqrt(fmax(0.0, (l2 * ((double)p.pd * 0.25) / (ip_resi * ip_resi) - 1.0) / (double)(p.pd - 1)));
     rec[p.words] = make_uint2(__float_as_uint(f_add), __float_as_uint(f_rescale));
     rec[p.words + 1] = make_uint2(cluster, 0u);
+    p.f_error[i] = (float)(2 * tmp_err);
   }
 }
 
@@ -1363,9 +1367,10 @@ int gpu_build_slimq_index(const float *base, size_t n, size_t dim, const hs_buil
   for (size_t i = 0; i < flip.size(); ++i) flip[i] = (uint8_t)(mix64(bp->seed * 0xD1B54A32D192ED03ull + i) >> 56);
   std::vector<float> rcent(num_cluster * pd);
   for (size_t c = 0; c < num_cluster; ++c) host_rotate(&cent[c * dim], dim, pd, td, flip.data(), &rcent[c * pd]);
-  DevBuf d_cent, d_rcent, d_flip, d_qrec;
+  DevBuf d_cent, d_rcent, d_flip, d_qrec, d_ferr;
   if ((rc = d_cent.alloc(cent.size() * 4)) != HS_OK || (rc = d_rcent.alloc(rcent.size() * 4)) != HS_OK ||
-      (rc = d_flip.alloc(flip.size())) != HS_OK || (rc = d_qrec.alloc(n * (words + 2) * 8)) != HS_OK)
+      (rc = d_flip.alloc(flip.size())) != HS_OK || (rc = d_qrec.alloc(n * (words + 2) * 8)) != HS_OK ||
+      (rc = d_ferr.alloc(n * 4)) != HS_OK)
     return fail(rc);
   if (cudaMemcpyAsync(d_cent.p, cent.data(), cent.size() * 4, cudaMemcpyHostToDevice, st) != cudaSuccess ||
       cudaMemcpyAsync(d_rcent.p, rcent.data(), rcent.size() * 4, cudaMemcpyHostToDevice, st) != cudaSuccess ||
@@ -1387,12 +1392,19 @@ int gpu_build_slimq_index(const float *base, size_t n, size_t dim, const hs_buil
   pp.flip = d_flip.as<uint8_t>();
   pp.fac = 1.0f / std::sqrt((float)td);
   pp.qrec = d_qrec.as<uint2>();
+  pp.f_error = d_ferr.as<float>();
   const size_t smem = 4 * pd * 4;
   if (cudaFuncSetAttribute(slimq_payload_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
     return fail(HS_ERR_CUDA);
   slimq_payload_kernel<<<(unsigned)((n + 3) / 4), 128, smem, st>>>(pp);
   if (cudaStreamSynchronize(st) != cudaSuccess || cudaGetLastError() != cudaSuccess) {
     set_error(std::string("slimq_payload_kernel: ") + cudaGetErrorString(cudaGetLastError()));
+    return fail(HS_ERR_CUDA);
+  }
+  // f_error stays on the host (hs_save_index writes it); d_ferr is freed on return
+  dg.h_f_error.resize(n);
+  if (cudaMemcpy(dg.h_f_error.data(), d_ferr.p, n * 4, cudaMemcpyDeviceToHost) != cudaSuccess) {
+    set_error(std::string("hs_build_slimq_index_gpu: f_error download: ") + cudaGetErrorString(cudaGetLastError()));
     return fail(HS_ERR_CUDA);
   }
   dg.kind = HS_KIND_SLIMQ;

@@ -299,6 +299,12 @@ int load_common(const uint8_t *bytes, size_t size, int kind, int metric, size_t 
     }
   }
   rc = build_index(g, metric, device, raw_base, out, capacity);
+  if (rc == HS_OK && kind == HS_KIND_SLIMQ) {
+    // kept on the host for hs_save_index: the traversal does not read them
+    (*out)->f_error = std::move(g.f_error);
+    (*out)->ex_bits = g.ex_bits;
+    (*out)->size_ex = g.size_data_per_element - 28 - (g.padded_dim_q / 8 + 12);   // checked by parse_graph
+  }
   if (rc == HS_OK && capacity > 0) {
     // the mirror of a patchable index: everything but the arrays that only the device needs
     g.mirror_only = true;
@@ -460,6 +466,9 @@ int hs::adopt_device_graph(DeviceGraph &dg, int device, hs_index **out) {
     ix->words = (uint32_t)(dg.padded_dim_q / 64);
     ix->trunc_dim = dg.trunc_dim;
     ix->t_const = slimq_default_tconst(dg.padded_dim_q, 3);
+    ix->f_error = std::move(dg.h_f_error);
+    ix->ex_bits = 3;                                    // as build_slimq_graph (data_layout.hpp)
+    ix->size_ex = dg.padded_dim_q * 3 / 8 + 8;
     I.padded_dim_q = dg.padded_dim_q;
     I.num_cluster = dg.num_cluster;
     bytes += dg.n * (dg.padded_dim_q / 64 + 2) * 8 + dg.num_cluster * dg.padded_dim_q * 4 + 4 * dg.padded_dim_q / 8;
@@ -1382,16 +1391,18 @@ int hs_debug_slimq_payload(const hs_index *ix, uint64_t *records, float *rotated
   return HS_OK;
 }
 
-// saveIndex (slim.h:717-751) of an HBM-resident hnsw_slim index: header, element records
-// [int32 level][uint32 total][uint64 label][8 stale pointer bytes][float vec[dim]], then per node
-// uint32 blob size + [uint16 offsets[level]][uint32 ids[total]].
+// saveIndex of an HBM-resident index: hnsw_slim (slim.h:717-751) — header, element records
+// [int32 level][uint32 total][uint64 label][8 stale pointer bytes][float vec[dim]] — or hnsw_slimq
+// (slimq.h:1161-1216, write_slimq_file in graph_build.cpp); then per node uint32 blob size +
+// [uint16 offsets[level]][uint32 ids[total]].  Labels are the device's 32-bit labels, zero-extended; the
+// pointer bytes are written as 0.
 int hs_save_index(hs_index *ix, const char *path) {
   if (!ix || !path) {
     set_error("null argument");
     return HS_ERR_ARG;
   }
-  if (ix->info.kind != HS_KIND_SLIM) {
-    set_error("hs_save_index: only hnsw_slim indices can be saved");
+  if (ix->info.kind != HS_KIND_SLIM && ix->info.kind != HS_KIND_SLIMQ) {
+    set_error("hs_save_index: only hnsw_slim and hnsw_slimq indices can be saved");
     return HS_ERR_UNSUPPORTED;
   }
   try {
@@ -1427,6 +1438,90 @@ int hs_save_index(hs_index *ix, const char *path) {
       *ids = row;
       return c;
     };
+    auto total_of = [&](size_t i, int lv) {
+      uint32_t total = 0;
+      const uint32_t *ids;
+      for (int l = 0; l <= lv; ++l) total += list(i, l, &ids);
+      return total;
+    };
+    auto write_blobs = [&](FILE *f) {
+      std::vector<uint8_t> blob;
+      bool ok = true;
+      for (size_t i = 0; i < n && ok; ++i) {
+        const int lv = level_of(i);
+        const uint32_t total = total_of(i, lv);
+        const uint32_t bsz = (uint32_t)(2 * lv + 4 * total);
+        ok &= std::fwrite(&bsz, 1, 4, f) == 4;
+        if (bsz == 0 || total == 0) continue;          // slim.h:741-748
+        blob.resize(bsz);
+        uint32_t run = 0;
+        size_t w = 2 * (size_t)lv;
+        const uint32_t *ids;
+        for (int l = 0; l <= lv; ++l) {
+          const uint32_t c = list(i, l, &ids);
+          std::memcpy(&blob[w], ids, 4 * (size_t)c);
+          w += 4 * (size_t)c;
+          run += c;
+          if (l < lv) {
+            const uint16_t o = (uint16_t)run;
+            std::memcpy(&blob[2 * l], &o, 2);
+          }
+        }
+        ok &= std::fwrite(blob.data(), 1, bsz, f) == bsz;
+      }
+      return ok;
+    };
+
+    if (I.kind == HS_KIND_SLIMQ) {
+      const size_t pd = I.padded_dim_q, words = pd / 64, rw = words + 2;
+      std::vector<float> cent(I.num_cluster * pd);
+      std::vector<uint8_t> flip(4 * pd / 8);
+      HS_CUDA(cudaMemcpy(cent.data(), ix->d_centroids, cent.size() * 4, cudaMemcpyDeviceToHost));
+      HS_CUDA(cudaMemcpy(flip.data(), ix->d_flip, flip.size(), cudaMemcpyDeviceToHost));
+      SlimqHead head;
+      head.n = n;
+      head.maxlevel = I.maxlevel;
+      head.threshold_level = I.threshold_level;
+      head.enterpoint = I.enterpoint;
+      head.maxM = I.maxM;
+      head.maxM0 = I.maxM0;
+      head.M = I.M;
+      head.ef_construction = I.ef_construction;
+      head.num_cluster = I.num_cluster;
+      head.dim = dim;
+      head.padded_dim = pd;
+      head.ex_bits = ix->ex_bits;
+      head.size_ex = ix->size_ex;
+      head.centroids = cent.data();
+      head.flip = flip.data();
+      std::vector<uint2> rec;
+      std::vector<uint64_t> code;
+      // the records streamed from the device in slabs; qrec holds each code word as (low half, high half)
+      return write_slimq_file(
+          path, head,
+          [&](size_t i0, size_t cnt, SlimqNode *out) -> int {
+            rec.resize(cnt * rw);
+            code.resize(cnt * words);
+            HS_CUDA(cudaMemcpy(rec.data(), ix->d_qrec + i0 * rw, rec.size() * 8, cudaMemcpyDeviceToHost));
+            for (size_t j = 0; j < cnt; ++j) {
+              const size_t i = i0 + j;
+              const uint2 *r = &rec[j * rw];
+              for (size_t w = 0; w < words; ++w) code[j * words + w] = (uint64_t)r[w].y << 32 | r[w].x;
+              SlimqNode &nd = out[j];
+              nd.level = level_of(i);
+              nd.total = total_of(i, nd.level);
+              nd.label = labels[i];
+              nd.cluster = r[words + 1].x;
+              nd.code = &code[j * words];
+              std::memcpy(&nd.f_add, &r[words].x, 4);
+              std::memcpy(&nd.f_rescale, &r[words].y, 4);
+              nd.f_error = ix->f_error[i];
+            }
+            return HS_OK;
+          },
+          write_blobs);
+    }
+
     FILE *f = std::fopen(path, "wb");
     if (!f) {
       set_error(std::string("cannot open ") + path + " for writing");
@@ -1454,9 +1549,7 @@ int hs_save_index(hs_index *ix, const char *path) {
       for (size_t j = 0; j < cnt && ok; ++j) {
         const size_t i = i0 + j;
         const int32_t lv = level_of(i);
-        uint32_t total = 0;
-        const uint32_t *ids;
-        for (int l = 0; l <= lv; ++l) total += list(i, l, &ids);
+        const uint32_t total = total_of(i, lv);
         const uint64_t label = labels[i], stale_ptr = 0;
         std::memcpy(&record[0], &lv, 4);
         std::memcpy(&record[4], &total, 4);
@@ -1466,30 +1559,7 @@ int hs_save_index(hs_index *ix, const char *path) {
         ok &= put(record.data(), rec);
       }
     }
-    std::vector<uint8_t> blob;
-    for (size_t i = 0; i < n && ok; ++i) {
-      const int lv = level_of(i);
-      uint32_t total = 0;
-      const uint32_t *ids;
-      for (int l = 0; l <= lv; ++l) total += list(i, l, &ids);
-      const uint32_t bsz = (uint32_t)(2 * lv + 4 * total);
-      ok &= put(&bsz, 4);
-      if (bsz == 0 || total == 0) continue;          // slim.h:741-748
-      blob.resize(bsz);
-      uint32_t run = 0;
-      size_t w = 2 * (size_t)lv;
-      for (int l = 0; l <= lv; ++l) {
-        const uint32_t c = list(i, l, &ids);
-        std::memcpy(&blob[w], ids, 4 * (size_t)c);
-        w += 4 * (size_t)c;
-        run += c;
-        if (l < lv) {
-          const uint16_t o = (uint16_t)run;
-          std::memcpy(&blob[2 * l], &o, 2);
-        }
-      }
-      ok &= put(blob.data(), bsz);
-    }
+    ok = ok && write_blobs(f);
     ok &= std::fclose(f) == 0;
     if (!ok) {
       set_error(std::string("write error on ") + path);

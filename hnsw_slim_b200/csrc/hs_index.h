@@ -5,6 +5,7 @@
 
 #include <memory>
 #include <mutex>
+#include <vector>
 
 #include "hs_internal.h"
 #include "traverse_fp32.cuh"
@@ -30,6 +31,9 @@ struct hs_index {
   float *d_centroids = nullptr;     // num_cluster x padded_dim (rotated)
   uint8_t *d_flip = nullptr;        // 4 * padded_dim / 8
   uint32_t words = 0, trunc_dim = 0;
+  // hnsw_slimq fields the file holds but the search does not read, kept on the host for hs_save_index
+  std::vector<float> f_error;       // n
+  uint64_t ex_bits = 0, size_ex = 0;
   uint32_t level_count[hs::kMaxLevels] = {};
   // delta patches (patch.cu): an index loaded with hs_load_reserve has rows for `capacity` nodes and keeps the
   // small host-side arrays (levels, upper-level slots and rows, labels) as a mirror; null / n otherwise
@@ -112,6 +116,7 @@ struct DeviceGraph {
   uint8_t *d_flip = nullptr;
   uint64_t padded_dim_q = 0, num_cluster = 0;
   uint32_t trunc_dim = 0;
+  std::vector<float> h_f_error;            // host, n entries; moved into the handle
 };
 int adopt_device_graph(DeviceGraph &dg, int device, hs_index **out);
 

@@ -2,6 +2,8 @@
 #pragma once
 #include <cstddef>
 #include <cstdint>
+#include <cstdio>
+#include <functional>
 #include <string>
 #include <utility>
 #include <vector>
@@ -136,6 +138,34 @@ int build_slimq_graph(const float *base, size_t n, size_t dim, size_t M, size_t 
                       size_t top_M, size_t low_m, int threads, uint64_t seed, const float *centroids,
                       size_t num_cluster, const uint32_t *cluster_ids, const uint64_t *labels,
                       const char *out_path);
+
+// HierarchicalNSWSlimQ::saveIndex's file (slimq.h:1161-1216), written by build_slimq_graph and hs_save_index.
+// Each element record is [int32 level][uint32 total][uint64 label][8 pointer bytes = 0][uint32 cluster @24]
+// [uint64 code[padded_dim / 64] @28, MSB-first][float f_add, f_rescale, f_error][ex block, size_ex bytes = 0].
+// The 3-bit ex-codes are not computed and the ex block is written as zeros: no search path reads it (SURVEY.md
+// App. A, only get_bin_est is called, slimq.h:737-738).
+struct SlimqHead {
+  uint64_t n = 0, maxM = 0, maxM0 = 0, M = 0, ef_construction = 0;
+  int32_t maxlevel = 0, threshold_level = 0;
+  uint32_t enterpoint = 0;
+  uint64_t num_cluster = 0, dim = 0, padded_dim = 0, ex_bits = 0, size_ex = 0;
+  const float *centroids = nullptr;    // num_cluster x padded_dim, rotated
+  const uint8_t *flip = nullptr;       // rotator sign bytes, 4 * padded_dim / 8
+};
+struct SlimqNode {
+  int32_t level = 0;
+  uint32_t total = 0;                  // neighbour ids over all of the node's levels
+  uint64_t label = 0;
+  uint32_t cluster = 0;
+  const uint64_t *code = nullptr;      // padded_dim / 64 words
+  float f_add = 0.f, f_rescale = 0.f, f_error = 0.f;
+};
+// Writes the header, the RaBitQ metadata, centroids, flip bytes and the n records to `path`, then the per-node
+// neighbour blobs through blobs(f).  nodes(i0, cnt, out) fills out[0, cnt) with nodes i0 .. i0 + cnt - 1, in slabs
+// of increasing i0; it returns HS_OK or an error code it has reported.  -> HS_OK, HS_ERR_IO or the nodes() code.
+int write_slimq_file(const char *path, const SlimqHead &h,
+                     const std::function<int(size_t i0, size_t cnt, SlimqNode *out)> &nodes,
+                     const std::function<bool(FILE *f)> &blobs);
 
 // pieces of the hnsw_slimq builder shared with the device builder (graph_gpu.cu)
 void host_rotate(const float *x, size_t dim, size_t pd, size_t td, const uint8_t *flip, float *out);

@@ -439,8 +439,15 @@ int hs_build_slimq_graph(const float *base, size_t n, size_t dim, const hs_build
  * point: ef_construction beam search + neighbour selection; reverse edges through one radix sort per
  * batch), so the graph is not the one a sequential build gives; its recall/cost is measured against the
  * host builder's in tests/test_gpu_build.py.  Needs 2 <= M <= 32, ef_construction <= 256.
- * hs_save_index writes any HBM-resident hnsw_slim index in saveIndex's format (slim.h:717-751): the
- * reference's loadIndex (and hs_load) read it. */
+ * hs_save_index writes an HBM-resident index, however it was built or loaded, in the reference's saveIndex
+ * format: hnsw_slim as HierarchicalNSWSlim::saveIndex (slim.h:717-751), hnsw_slimq as
+ * HierarchicalNSWSlimQ::saveIndex (slimq.h:1161-1216).  The reference's loadIndex and hs_load read the file.
+ * Labels are the index's 32-bit labels, zero-extended; the 8 pointer bytes of every record are written as 0.
+ * An hnsw_slimq record keeps its code, f_add, f_rescale and f_error, but its 3-bit ex-code block is written
+ * as zeros (no search path reads it, as for hs_build_slimq_graph), so a reference-built file comes back with
+ * zero ex blocks.  The file holds no raw rows: hs_load of a saved hnsw_slimq file needs the same raw rows, in
+ * the same order, for the exact rerank — for a GPU-built index, the rows given to hs_build_slimq_index_gpu.
+ * HS_KIND_HNSW indices give HS_ERR_UNSUPPORTED; a file that cannot be written gives HS_ERR_IO. */
 int hs_build_slim_index_gpu(const float *base, size_t n, size_t dim, int metric, const hs_build_params *p,
                             const uint64_t *labels, int device, hs_index **out);
 int hs_save_index(hs_index *, const char *out_graph_path);
