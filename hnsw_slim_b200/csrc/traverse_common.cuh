@@ -5,6 +5,7 @@
 #include <cuda_runtime.h>
 
 #include <cstdint>
+#include <type_traits>
 
 #include "hs_internal.h"
 
@@ -125,6 +126,71 @@ __device__ __forceinline__ float eval_rows_reg(const float4 *__restrict__ vec, u
   return my_d;
 }
 
+// Query chunk j of lane t of a team for eval_rows_ring: Q is either `float4[CPL]` (registers, as in eval_rows_reg) or
+// `float4 *` (the query's chunks in shared memory, as in eval_rows_sq).
+template <typename Q>
+__device__ __forceinline__ float4 query_chunk(const Q &q, int j, int t) {
+  if constexpr (std::is_pointer_v<Q>) return q[8 * j + t];
+  else return q[j];
+}
+
+// One round of eval_rows_sq: G groups of 4 rows from row 4 * it0 on, each group with at least one row.  The loads of
+// all G groups are issued before the first FMA.  A team without a row of its own re-reads the last row (an address
+// its group loads anyway) instead of skipping its loads: loads that happen on some paths only leave the rows
+// conditionally defined, and the kernel then spills hundreds of bytes.  Its sum is replaced by 0, as in eval_rows_reg.
+// The query chunk is read with a volatile LDS.128 next to its FMAs: hoisted above the row loads, the chunks take the
+// registers of the second group and ptxas delays that group's loads behind the first group's FMAs.
+template <int CPL, int METRIC, int G>
+__device__ __forceinline__ void eval_round_sq(const float4 *__restrict__ vec, uint32_t row_chunks, const float4 *qs,
+                                              uint32_t my_id, int count, int it0, int lane, float &my_d) {
+  const int team = lane >> 3, t = lane & 7;
+  float4 x[G][CPL];
+#pragma unroll
+  for (int g = 0; g < G; ++g) {
+    const uint32_t id = __shfl_sync(FULL, my_id, min((it0 + g) * 4 + team, count - 1));
+    const float4 *row = vec + (size_t)id * row_chunks + t;
+#pragma unroll
+    for (int j = 0; j < CPL; ++j) x[g][j] = __ldg(row + 8 * j);
+  }
+  acc2_t acc2[G];
+#pragma unroll
+  for (int g = 0; g < G; ++g) acc2[g] = 0ull;
+#pragma unroll
+  for (int j = 0; j < CPL; ++j) {
+    float4 qj;
+    const unsigned a = (unsigned)__cvta_generic_to_shared(qs + 8 * j + t);
+    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(qj.x), "=f"(qj.y), "=f"(qj.z), "=f"(qj.w) : "r"(a));
+#pragma unroll
+    for (int g = 0; g < G; ++g) acc2[g] = acc4<METRIC>(acc2[g], qj, x[g][j]);
+  }
+#pragma unroll
+  for (int g = 0; g < G; ++g) {
+    const float acc = team_reduce(sum2((it0 + g) * 4 + team < count ? acc2[g] : 0ull));
+    const float v = __shfl_sync(FULL, acc, (lane & 3) * 8);
+    if ((lane >> 2) == it0 + g) my_d = finish<METRIC>(v);
+  }
+}
+
+// Same as eval_rows_reg with the query in shared memory (`qs`: the query's row_chunks chunks; the four teams read the
+// same 16 bytes, a broadcast, and a team reads 128 contiguous bytes, so a chunk is one conflict-free LDS.128).  That
+// frees the 4 x CPL query registers for a second row group: U x 4 rows in flight per warp, so a hop of up to 8 fresh
+// rows (U = 2) waits for one round of row loads instead of two.  Rounds of U groups while more than U - 1 groups of
+// rows are left, then single groups.  Every group keeps its own FFMA2 chain in chunk order: the sums do not depend on
+// U or on where the query is read from (bit-identical to eval_rows_reg).
+template <int CPL, int METRIC, int U>
+__device__ __forceinline__ float eval_rows_sq(const float4 *__restrict__ vec, uint32_t row_chunks, const float4 *qs,
+                                              uint32_t my_id, int count, int lane) {
+  float my_d = 0.f;
+  int it0 = 0;
+  if constexpr (U > 1) {
+#pragma unroll 1
+    for (; count - it0 * 4 > 4 * (U - 1); it0 += U) eval_round_sq<CPL, METRIC, U>(vec, row_chunks, qs, my_id, count, it0, lane, my_d);
+  }
+#pragma unroll 1
+  for (; it0 * 4 < count; ++it0) eval_round_sq<CPL, METRIC, 1>(vec, row_chunks, qs, my_id, count, it0, lane, my_d);
+  return my_d;
+}
+
 // Same through a per-warp shared-memory ring of R rows (R a multiple of 4): ALL rows of a chunk are put in flight at
 // once with 16-byte cp.async copies (one per lane and row: a row of CPL x 8 chunks is at most 32 of them), then
 // scored out of shared memory — the rows-in-flight count no longer depends on the register budget, and a hop waits
@@ -133,10 +199,9 @@ __device__ __forceinline__ void cp_async16(void *smem_dst, const void *gsrc) {
   const unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d), "l"(gsrc) : "memory");
 }
-template <int CPL, int METRIC, int R>
-__device__ __forceinline__ float eval_rows_ring(const float4 *__restrict__ vec, uint32_t row_chunks,
-                                                const float4 (&q)[CPL], float4 *ring, uint32_t my_id, int count,
-                                                int lane) {
+template <int CPL, int METRIC, int R, typename Q>
+__device__ __forceinline__ float eval_rows_ring(const float4 *__restrict__ vec, uint32_t row_chunks, const Q &q,
+                                                float4 *ring, uint32_t my_id, int count, int lane) {
   static_assert(R % 4 == 0 && R > 0, "ring rows must be a multiple of 4");
   const int team = lane >> 3, t = lane & 7;
   float my_d = 0.f;
@@ -155,7 +220,7 @@ __device__ __forceinline__ float eval_rows_ring(const float4 *__restrict__ vec, 
       if (src < n) {
         const float4 *row = ring + src * (CPL * 8) + t;
 #pragma unroll
-        for (int j = 0; j < CPL; ++j) acc2 = acc4<METRIC>(acc2, q[j], row[8 * j]);
+        for (int j = 0; j < CPL; ++j) acc2 = acc4<METRIC>(acc2, query_chunk(q, j, t), row[8 * j]);
       }
       const float acc = team_reduce(sum2(acc2));
       const float v = __shfl_sync(FULL, acc, (lane & 3) * 8);

@@ -54,7 +54,7 @@ namespace {
 #define HS_TRAVERSE_MIN_CTAS_BIG 6 // same for the pools of 5..8 register slots per lane (ef 129..256)
 #endif
 #ifndef HS_TRAVERSE_U
-#define HS_TRAVERSE_U 1            // x4 rows whose loads are in flight per warp
+#define HS_TRAVERSE_U 2            // x4 rows whose loads are in flight per warp (kernels with the query in shared memory)
 #endif
 #ifndef HS_ROW_RING
 #define HS_ROW_RING 0              // > 0: rows go through a shared-memory ring of this many rows (cp.async), see eval_rows_ring
@@ -67,6 +67,13 @@ template <int SLOTS> struct PoolSel {
   using type = std::conditional_t<(SLOTS >= 5 && HS_POOL_COMPACT), RegPool32C<SLOTS>, RegPool32<SLOTS>>;
 };
 template <> struct PoolSel<0> { using type = SmemPool; };
+
+// Where a kernel keeps the query.  Shared memory for the generic path (CPL 0) and for the ef <= 128 register pools
+// (2 / 4 slots): there the 4 x CPL query registers per lane pay for a second row group in eval_rows_sq (8 rows in
+// flight instead of 4), which turns the 2 to 3 load rounds of a typical hop (about 9 fresh rows at ef = 100) into 1
+// to 2.  Registers for CPL 3 / 4 with the larger pools (5..8 slots, ef 129..256) and the shared-memory pool: those
+// keep 4 rows in flight.  plan_traverse sizes the shared-memory carve-out by the same rule.
+constexpr bool query_in_smem(int cpl, int slots) { return cpl == 0 || slots == 2 || slots == 4; }
 
 template <int CPL, int METRIC, int SLOTS>
 __global__ void __launch_bounds__(128, SLOTS >= 5 ? HS_TRAVERSE_MIN_CTAS_BIG : HS_TRAVERSE_MIN_CTAS)
@@ -87,6 +94,7 @@ traverse_kernel(const __grid_constant__ TraverseParams p) {
   }
   uint32_t *stage_ids = reinterpret_cast<uint32_t *>(wbase + p.off_stage);
   uint32_t *ghosts = stage_ids + 32;        // 16 words: exact-tie side list (traverse_common.cuh ghost_append)
+  constexpr bool QSMEM = query_in_smem(CPL, SLOTS);
   float4 *qs = reinterpret_cast<float4 *>(wbase + p.off_query);
 
   if (p.overlap) {
@@ -142,10 +150,11 @@ traverse_kernel(const __grid_constant__ TraverseParams p) {
       acked = true;
     }
 
-    // ---- query: lane t of each team owns chunks t, t+8, ... (zero-padded past dim).  Each
-    //      chunk is read ONCE per warp (one 16-byte load per lane when the batch is 16-byte
-    //      aligned) and handed to the four teams by shuffles: the batch may sit in pinned host
-    //      memory (zero-copy hs_search_batch), where every request crosses PCIe ----
+    // ---- query (zero-padded past dim): each chunk is read ONCE per warp (one 16-byte load per
+    //      lane when the batch is 16-byte aligned): the batch may sit in pinned host memory
+    //      (zero-copy hs_search_batch), where every request crosses PCIe.  Into shared memory
+    //      (QSMEM), or into registers, where lane t of each team owns chunks t, t+8, ... and the
+    //      chunks are handed to the four teams by shuffles ----
     const float *qptr = p.queries + (size_t)qi * p.dim;
     auto load_chunk = [&](uint32_t ch) -> float4 {
       const uint32_t c = 4u * ch;
@@ -161,7 +170,7 @@ traverse_kernel(const __grid_constant__ TraverseParams p) {
       return v;
     };
     float4 q[QN];
-    if (CPL > 0) {
+    if constexpr (!QSMEM) {
       const float4 mine = load_chunk((uint32_t)lane);      // row_chunks = 8 * CPL <= 32
 #pragma unroll
       for (int j = 0; j < QN; ++j) {
@@ -179,10 +188,14 @@ traverse_kernel(const __grid_constant__ TraverseParams p) {
 
     auto eval = [&](uint32_t my_id, int count) -> float {
       if constexpr (CPL > 0) {
+        const float4 *qsm = qs;
 #if HS_ROW_RING > 0
-        return eval_rows_ring<QN, METRIC, HS_ROW_RING>(p.vec, p.row_chunks, q, qs, my_id, count, lane);
+        float4 *ring = qs + (QSMEM ? p.row_chunks : 0u);      // the ring follows the query (plan_traverse)
+        if constexpr (QSMEM) return eval_rows_ring<QN, METRIC, HS_ROW_RING>(p.vec, p.row_chunks, qsm, ring, my_id, count, lane);
+        else return eval_rows_ring<QN, METRIC, HS_ROW_RING>(p.vec, p.row_chunks, q, ring, my_id, count, lane);
 #else
-        return eval_rows_reg<QN, METRIC, HS_TRAVERSE_U>(p.vec, p.row_chunks, q, my_id, count, lane);
+        if constexpr (QSMEM) return eval_rows_sq<QN, METRIC, HS_TRAVERSE_U>(p.vec, p.row_chunks, qsm, my_id, count, lane);
+        else return eval_rows_reg<QN, METRIC, 1>(p.vec, p.row_chunks, q, my_id, count, lane);
 #endif
       } else {
         return eval_rows_smem<METRIC>(p.vec, p.row_chunks, qs, my_id, count, lane);
@@ -537,8 +550,10 @@ int plan_traverse(TraverseParams &p, int metric, int hash_bits_override, int gha
   const int met = metric == HS_METRIC_IP ? HS_METRIC_IP : HS_METRIC_L2;
   const uint32_t list_bytes = slv ? 0u : align_up(p.ef * 8u, 16);
   const uint32_t stage_bytes = 32 * 4 + 16 * 4;       // staging ids + the exact-tie side list
-  // large dims: the query; small dims with HS_ROW_RING: the row ring (same carve-out, off_query)
-  const uint32_t query_bytes = cplv == 0 ? p.row_chunks * 16u : (uint32_t)HS_ROW_RING * p.row_chunks * 16u;
+  // the query where the kernel reads it from shared memory (query_in_smem), then, small dims with HS_ROW_RING, the
+  // row ring (same carve-out, off_query)
+  const uint32_t query_bytes = (query_in_smem(cplv, slv) ? p.row_chunks * 16u : 0u)
+                               + (cplv == 0 ? 0u : (uint32_t)HS_ROW_RING * p.row_chunks * 16u);
 
   // Shared-memory tables first.  They bound the resident warps: 24 per SM (what the register file
   // allows) needs <= 9.4 KB per warp.  When the table of this ef (plus the query of a large dim)
